@@ -13,6 +13,7 @@ from rank 0 over NCCL at session build, no steady-state communication.
 import argparse
 import json
 import os
+import re
 import sys
 import threading
 import time
@@ -22,6 +23,7 @@ sys.path.insert(0, ROOT)
 
 MODEL = os.path.join(ROOT, "tests", "golden", "mbv2_int8.mnn")
 BATCH_PER_GPU = 32
+DUMP_ELEMENTS_PER_LAYER = 1 << 18     # --dump-outputs: 36 layers x 1 MB of float32 at most
 # one metric string and one workload string for BOTH arms (the driver divides the two lines only when they agree)
 METRIC = "inferences/sec (MobileNet-v2-int8 224x224, batch 32 per GPU, dense int8 conv path)"
 WORKLOAD = ("MobileNet-v2 int8 .mnn (reference Revert-quantised graph, retuned weights), batch 32 per GPU, the 36 dense int8 "
@@ -172,11 +174,11 @@ def cpu_reference_rate(batch, iters, warmup, threads=None):
 def plugin_e2e_rate(batch=BATCH_PER_GPU, warmup=5, iters=20, windows=9, device=None, pin_user_tensors=True):
     """The WHOLE .mnn through the reference's own Interpreter::runSession (copyFromHostTensor of the fp32 NCHW input +
     runSession + copyToHostTensor of the result per iteration, benchmark/benchmark.cpp:120-181 style) scheduled on
-    MNN_FORWARD_CUDA = mnn_b200/libmnn_b200_plugin.so: the call a user of MNN makes.  The host program is the reference core
+    MNN_FORWARD_CUDA = oracle/_ref/libmnn_b200_plugin.so: the call a user of MNN makes.  The host program is the reference core
     built under oracle/_ref (the CALLER of the plugin, not a checker).  Median of `windows` windows of `iters` iterations."""
     import subprocess
     from oracle import oracle as O
-    plugin = os.path.join(ROOT, "mnn_b200", "libmnn_b200_plugin.so")
+    plugin = O.PLUGIN
     if not (O.have_reference() and os.path.exists(plugin)):
         return {"value": None, "note": "reference core or plugin .so not present"}
     env = dict(os.environ, REFDUMP_PLUGIN=plugin, REFDUMP_BENCH_WINDOWS=str(windows))
@@ -203,6 +205,22 @@ def plugin_e2e_rate(batch=BATCH_PER_GPU, warmup=5, iters=20, windows=9, device=N
             "h2d_bytes_per_step": j.get("h2d_bytes"), "d2h_bytes_per_step": j.get("d2h_bytes"),
             "host_tensors": "pinned in place (MNNB200_PLUGIN_HOSTREG=1)" if pin_user_tensors else "pageable (plugin default)",
             "note": "unmodified MNN Interpreter + libmnn_b200_plugin.so, host tensors in/out every iteration, every command on the GPU"}
+
+
+def dump_outputs(sess, out_dir):
+    """The int8 output of every dense conv of the session's last step, as out_dir/<layer>_<name>.npy in float32 (logical NCHW).
+    A layer with more than DUMP_ELEMENTS_PER_LAYER elements is written as the elements at a fixed, seeded sample of its flat
+    NCHW positions (np.random.default_rng(layer).integers(0, size, DUMP_ELEMENTS_PER_LAYER), sorted)."""
+    import numpy as np
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    sess.stream.synchronize()
+    for i, (node, _, _, y) in enumerate(sess.layers):
+        with torch.cuda.stream(sess.stream):
+            out = sess.backend.onCopyBuffer(y, "same").astype(np.float32).ravel()
+        if out.size > DUMP_ELEMENTS_PER_LAYER:
+            out = out[np.sort(np.random.default_rng(i).integers(0, out.size, DUMP_ELEMENTS_PER_LAYER))]
+        np.save(os.path.join(out_dir, f"{i:02d}_{re.sub(r'[^A-Za-z0-9_.-]', '_', node.name)}.npy"), out)
 
 
 def run_reference(args, rank):
@@ -267,7 +285,11 @@ def main():
                     help="mbv2 = the driver's line (BASELINE configs[1]); resnet_wino / qwen = configs[2] / configs[3] alone")
     ap.add_argument("--wino-unit", type=int, default=6, choices=[2, 4, 6])
     ap.add_argument("--qwen-layers", type=int, default=24)
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one computed (every conv's output) to DIR/*.npy")
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl == "reference" or args.workload != "mbv2"):
+        ap.error("--dump-outputs writes the outputs of the CUDA arm's mbv2 workload only")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -325,6 +347,8 @@ def main():
         ev1.record()
     barrier()
     my_ms = ev0.elapsed_time(ev1)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(sess, args.dump_outputs)
     ms_total = _max_over_ranks(torch, dist, world, my_ms)
     # a longer look at the same loop (several K-step windows, >= 0.25 s): the median window guards the short K-step region
     # against one straggling host-side graph launch (round-1 SCALE N=4 dip)

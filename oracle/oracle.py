@@ -4,6 +4,7 @@ TEST INFRASTRUCTURE ONLY: importable from tests/, __graft_entry__.smoke() and be
 cpu_baseline / --impl reference leg.  mnn_b200 (the product) never imports this module.
 """
 import ctypes as C
+import hashlib
 import os
 import struct
 import subprocess
@@ -15,6 +16,9 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(HERE, "libmnn_oracle.so")
 REF_DIR = os.path.join(HERE, "_ref")
 REFDUMP = os.path.join(REF_DIR, "refdump")
+# the MNN_FORWARD_CUDA plugin (product code, mnn_b200/csrc/plugin) is compiled against the reference's headers, so it is built
+# where the reference is and kept beside the core library that hosts it
+PLUGIN = os.path.join(REF_DIR, "libmnn_b200_plugin.so")
 
 
 def build(force=False):
@@ -219,11 +223,42 @@ def have_reference():
     return os.path.exists(REFDUMP) and os.path.exists(os.path.join(REF_DIR, "libMNN.so"))
 
 
-def _run_refdump(args, timeout=600):
+def _run_refdump(args, timeout=600, exe=REFDUMP):
     env = dict(os.environ)
     env["LD_LIBRARY_PATH"] = REF_DIR + ":" + env.get("LD_LIBRARY_PATH", "")
-    return subprocess.run([REFDUMP] + [str(a) for a in args], env=env, capture_output=True, text=True,
+    return subprocess.run([exe] + [str(a) for a in args], env=env, capture_output=True, text=True,
                           timeout=timeout, check=True)
+
+
+# Answers of the reference harness, recorded by tests/golden/make_golden.py and keyed by the request they answer, so that the
+# comparisons with the reference hold on machines without the reference build (where it is built, it answers live).
+RECORDED = os.path.join(os.path.dirname(HERE), "tests", "golden", "reference_calls.npz")
+_recorded = None
+recording = None     # make_golden.py sets a dict here: every answer of the live reference is kept in it under its request key
+
+
+def _reference_answer(exe, args, payload):
+    """The bytes `exe cmd req.bin out.bin *rest` writes for args = [cmd, *rest] and req.bin = payload: from the live reference when
+    oracle/_ref holds it, else the answer recorded for the same request."""
+    global _recorded
+    key = hashlib.sha256(repr([os.path.basename(exe)] + [str(a) for a in args]).encode() + payload).hexdigest()[:32]
+    if not os.path.exists(exe):
+        if _recorded is None:
+            _recorded = dict(np.load(RECORDED)) if os.path.exists(RECORDED) else {}
+        if key in _recorded:
+            return _recorded[key].tobytes()
+        raise FileNotFoundError(f"no recorded reference answer for this '{args[0]}' request and {exe} is not built: "
+                                "build the reference (oracle/build_ref.py) or re-record (tests/golden/make_golden.py calls)")
+    with tempfile.TemporaryDirectory() as d:
+        req, out = os.path.join(d, "req.bin"), os.path.join(d, "out.bin")
+        with open(req, "wb") as f:
+            f.write(payload)
+        _run_refdump([args[0], req, out] + list(args[1:]), exe=exe)
+        with open(out, "rb") as f:
+            raw = f.read()
+    if recording is not None:
+        recording[key] = np.frombuffer(raw, np.uint8)
+    return raw
 
 
 def ref_conv(mode, x, w, bias, scale, stride=(1, 1), pad=(0, 0), dilate=(1, 1), group=1, relu=False,
@@ -238,12 +273,7 @@ def ref_conv(mode, x, w, bias, scale, stride=(1, 1), pad=(0, 0), dilate=(1, 1), 
                       dilate[0], dilate[1], group, int(relu), z_in, z_out, min_v, max_v, scale_in, scale_out)
     b = np.ascontiguousarray(bias, np.int32 if mode == 0 else np.float32)
     s = np.ascontiguousarray(scale, np.float32)
-    with tempfile.TemporaryDirectory() as d:
-        req, out = os.path.join(d, "req.bin"), os.path.join(d, "out.bin")
-        with open(req, "wb") as f:
-            f.write(hdr + x.tobytes() + w.tobytes() + b.tobytes() + s.tobytes())
-        _run_refdump(["conv", req, out])
-        raw = open(out, "rb").read()
+    raw = _reference_answer(REFDUMP, ["conv"], hdr + x.tobytes() + w.tobytes() + b.tobytes() + s.tobytes())
     dims = struct.unpack("<4i", raw[:16])
     return np.frombuffer(raw[16:], np.int8).reshape(dims).copy()
 
@@ -258,11 +288,7 @@ def ref_linear(x, wq, alpha, asym=False, bias=None, relu=False, relu6=False, thr
     payload = hdr + x.tobytes() + wq.tobytes() + np.ascontiguousarray(alpha, np.float32).tobytes()
     if bias is not None:
         payload += np.ascontiguousarray(bias, np.float32).tobytes()
-    with tempfile.TemporaryDirectory() as d:
-        req, out = os.path.join(d, "req.bin"), os.path.join(d, "out.bin")
-        open(req, "wb").write(payload)
-        _run_refdump(["linear", req, out, threads])
-        return np.fromfile(out, np.float32).reshape(tokens, oc)
+    return np.frombuffer(_reference_answer(REFDUMP, ["linear", threads], payload), np.float32).reshape(tokens, oc).copy()
 
 
 def ref_run_model(model, batch, seed, outdir, threads=1):
@@ -345,13 +371,7 @@ def ref_wino(x, w, wscale, bias, in_scales, in_zeros, w_scales, unit, pad=1, s_i
     hdr = struct.pack("<13i2f", n, ic, ih, iw, oc, r, pad, unit, int(relu), z_in, z_out, clamp_min, clamp_max, s_in, s_out)
     payload = hdr + x.tobytes() + w.tobytes() + bias.tobytes() + wscale.tobytes() + in_scales.tobytes() + \
         in_zeros.tobytes() + w_scales.tobytes()
-    env = dict(os.environ)
-    env["LD_LIBRARY_PATH"] = REF_DIR + ":" + env.get("LD_LIBRARY_PATH", "")
-    with tempfile.TemporaryDirectory() as d:
-        req, out = os.path.join(d, "req.bin"), os.path.join(d, "out.bin")
-        open(req, "wb").write(payload)
-        subprocess.run([REFDUMP_AVX2, "wino", req, out], env=env, capture_output=True, text=True, timeout=600, check=True)
-        raw = open(out, "rb").read()
+    raw = _reference_answer(REFDUMP_AVX2, ["wino"], payload)
     dims = struct.unpack("<4i", raw[:16])
     return np.frombuffer(raw[16:], np.int8).reshape(dims).copy()
 
@@ -393,11 +413,8 @@ def ref_matmul(a, b, transpose_a=False, transpose_b=False):
     e, l = (a3.shape[2], a3.shape[1]) if transpose_a else (a3.shape[1], a3.shape[2])
     h = b3.shape[1] if transpose_b else b3.shape[2]
     hdr = struct.pack("<8i", batch, e, l, h, int(transpose_a), int(transpose_b), 0, 0)
-    with tempfile.TemporaryDirectory() as d:
-        req, out = os.path.join(d, "req.bin"), os.path.join(d, "out.bin")
-        open(req, "wb").write(hdr + a3.tobytes() + b3.tobytes())
-        _run_refdump(["matmul", req, out])
-        return np.fromfile(out, np.float32).reshape(a.shape[:-2] + (e, h))
+    raw = _reference_answer(REFDUMP, ["matmul"], hdr + a3.tobytes() + b3.tobytes())
+    return np.frombuffer(raw, np.float32).reshape(a.shape[:-2] + (e, h)).copy()
 
 
 # --------------------------------------------------------------------------------------------
@@ -417,11 +434,7 @@ def ref_pool_int8(x, kernel, stride, pad, is_avg, scale=0.05, zero=0):
     x = np.ascontiguousarray(x, np.int8)
     n, c, ih, iw = x.shape
     hdr = struct.pack("<12if", n, c, ih, iw, kernel[0], kernel[1], stride[0], stride[1], pad[0], pad[1], int(is_avg), int(zero), scale)
-    with tempfile.TemporaryDirectory() as d:
-        req, out = os.path.join(d, "req.bin"), os.path.join(d, "out.bin")
-        open(req, "wb").write(hdr + x.tobytes())
-        _run_refdump(["pool", req, out])
-        raw = open(out, "rb").read()
+    raw = _reference_answer(REFDUMP, ["pool"], hdr + x.tobytes())
     dims = struct.unpack("<4i", raw[:16])
     return np.frombuffer(raw[16:], np.int8).reshape(dims).copy()
 

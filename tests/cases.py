@@ -5,6 +5,8 @@ test/op/ConvInt8Test.cpp:175-207 (x[i] = i % 255 - 127, w = (i^2+j^2+k^2) % 255 
 bias = (10000 + i*i*10 - i*i*i) % 12580, scale = ((127-i)*i % 128) / 20000), so the same vectors the
 reference test feeds to its CPU backend are fed to the oracle and to the CUDA path.
 """
+import os
+
 import numpy as np
 
 
@@ -106,3 +108,64 @@ def wino_oracle(O, c, unit, fn=None):
     fn = fn or O.wino_conv_int8
     return fn(c["x"], c["w"], c["ws"], c["bias"], c["in_scales"], c["in_zeros"], c["w_scales"], unit, c["pad"], c["s_in"],
               c["z_in"], c["s_out"], c["z_out"], -127, 127, c["relu"])
+
+
+def refdump_input(shape, seed):
+    """The fp32 input `refdump run` feeds a model (oracle/refdump.cpp fillInput): std::mt19937(seed) through
+    uniform_real_distribution<float>(-1, 1) in NCHW order.  RandomState(seed) draws the same 32-bit words."""
+    words = np.random.RandomState(seed).randint(0, 2 ** 32, int(np.prod(shape)), dtype=np.uint64)
+    u = words.astype(np.float32) / np.float32(2 ** 32)
+    u = np.where(u >= 1, np.nextafter(np.float32(1), np.float32(0)), u).astype(np.float32)
+    return (u * np.float32(2) + np.float32(-1)).reshape(shape)
+
+
+# ---- inputs of golden files that are regenerated from their seeds instead of stored (stored, they would take the files past
+# 1 MB); tests/golden/make_golden.py draws them through the same functions ---------------------------------------------------
+GOLD = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
+DW_CASES = [(32, 3, 2, 16, 16, (1, 1), (1, 1), 1), (96, 3, 1, 15, 15, (2, 2), (1, 1), 1), (40, 5, 1, 9, 11, (1, 1), (2, 2), 0),
+            (7, 3, 3, 6, 6, (1, 1), (0, 0), 1)]
+# the last five: ONE token = the decode step, where the reference switches to its single-quant arithmetic (asymmetric input
+# quantisation over the row incl. the pack padding, zero point folded into the bias; ConvInt8TiledExecutor.cpp:1033, 1432, 2016-2050)
+LINEAR_CASES = [(8, 64, 48, False, True, -1, 1), (33, 256, 200, True, True, -1, 1), (5, 96, 33, False, False, -1, 1),
+                (64, 512, 128, True, False, -1, 1), (1, 2048, 512, True, True, -1, 1), (1, 100, 64, False, False, 0.2, 1.0),
+                (1, 250, 33, True, False, -1, -0.1), (1, 320, 200, True, True, -3, 5), (1, 64, 48, False, True, 0.25, 0.25)]
+
+
+def dw_linear_inputs():
+    rng = np.random.default_rng(77)
+    out = {}
+    for i, (ch, k, n, ih, iw, st, pad, relu) in enumerate(DW_CASES):
+        x = rng.integers(-128, 128, (n, ch, ih, iw)).astype(np.int8)
+        w = rng.integers(-127, 128, (ch, 1, k, k)).astype(np.int8)
+        s_in, s_out = 0.043, 0.061
+        z_in, z_out = int(rng.integers(-4, 5)), int(rng.integers(-4, 5))
+        ws = (rng.uniform(0.003, 0.012, ch) / k * s_out / s_in).astype(np.float32)
+        bias = (rng.uniform(-1, 1, ch) * 10 * s_out).astype(np.float32)
+        out.update({f"d{i}_x": x, f"d{i}_w": w, f"d{i}_ws": ws, f"d{i}_bias": bias, f"d{i}_stride": np.array(st),
+                    f"d{i}_pad": np.array(pad), f"d{i}_relu": np.array(relu), f"d{i}_q": np.array([s_in, z_in, s_out, z_out])})
+    for j, (tokens, ic, oc, asym, hb, lo, hi) in enumerate(LINEAR_CASES):
+        x = rng.uniform(lo, hi, (tokens, ic)).astype(np.float32)
+        wq = rng.integers(-128, 128, (oc, ic)).astype(np.int8)
+        alpha = rng.uniform(0.001, 0.01, oc).astype(np.float32)
+        wmin = rng.uniform(-0.05, 0.05, oc).astype(np.float32) if asym else np.zeros(0, np.float32)
+        bias = rng.uniform(-1, 1, oc).astype(np.float32) if hb else np.zeros(0, np.float32)
+        out.update({f"l{j}_x": x, f"l{j}_wq": wq, f"l{j}_alpha": alpha, f"l{j}_wmin": wmin, f"l{j}_bias": bias})
+    return out
+
+
+def matmul_inputs():
+    from tests.test_matmul import CASES, make
+    rng = np.random.default_rng(808)
+    out = {}
+    for i, (bd, e, l, h, ta, tb) in enumerate(CASES):
+        a, b = make(rng, bd, e, l, h, ta, tb)
+        out.update({f"m{i}_a": a, f"m{i}_b": b, f"m{i}_ta": np.array(ta), f"m{i}_tb": np.array(tb)})
+    return out
+
+
+def load_golden(name):
+    """tests/golden/<name>.npz (the reference's outputs) together with the inputs regenerated for it"""
+    g = np.load(os.path.join(GOLD, name + ".npz"))
+    inputs = {"dw_linear_golden": dw_linear_inputs, "matmul_golden": matmul_inputs,
+              "mbv2_int8_checkpoints": lambda: {"input": refdump_input((1, 3, 224, 224), 7)}}[name]()
+    return dict(inputs, **{k: g[k] for k in g.files})

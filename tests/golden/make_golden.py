@@ -10,7 +10,7 @@ import numpy as np
 ROOT = os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 sys.path.insert(0, ROOT)
 from oracle import oracle as O  # noqa: E402
-from tests.cases import KAT_SWEEP, kat_conv, random_modern_case  # noqa: E402
+from tests.cases import DW_CASES, KAT_SWEEP, LINEAR_CASES, dw_linear_inputs, kat_conv, matmul_inputs, random_modern_case, refdump_input  # noqa: E402,E501
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 
@@ -51,44 +51,20 @@ def conv_golden():
 
 
 def dw_linear_golden():
-    """depthwise int8 conv + dynamic-quant linear outputs from the real reference (refdump conv mode 1 / linear)."""
-    rng = np.random.default_rng(77)
-    out = {}
-    i = 0
-    for (ch, k, n, ih, iw, st, pad, relu) in [(32, 3, 2, 16, 16, (1, 1), (1, 1), 1), (96, 3, 1, 15, 15, (2, 2), (1, 1), 1),
-                                              (40, 5, 1, 9, 11, (1, 1), (2, 2), 0), (7, 3, 3, 6, 6, (1, 1), (0, 0), 1)]:
-        x = rng.integers(-128, 128, (n, ch, ih, iw)).astype(np.int8)
-        w = rng.integers(-127, 128, (ch, 1, k, k)).astype(np.int8)
-        s_in, s_out = 0.043, 0.061
-        z_in, z_out = int(rng.integers(-4, 5)), int(rng.integers(-4, 5))
-        ws = (rng.uniform(0.003, 0.012, ch) / k * s_out / s_in).astype(np.float32)
-        bias = (rng.uniform(-1, 1, ch) * 10 * s_out).astype(np.float32)
-        y = O.ref_conv(1, x, w, bias, ws, stride=st, pad=pad, group=ch, relu=relu, z_in=z_in, z_out=z_out,
-                       scale_in=s_in, scale_out=s_out)
-        out.update({f"d{i}_x": x, f"d{i}_w": w, f"d{i}_ws": ws, f"d{i}_bias": bias, f"d{i}_stride": st, f"d{i}_pad": pad,
-                    f"d{i}_relu": relu, f"d{i}_q": np.array([s_in, z_in, s_out, z_out], np.float64), f"d{i}_y": y})
-        i += 1
-    out["ndw"] = i
-    j = 0
-    # the last five: ONE token = the decode step, where the reference switches to its single-quant arithmetic (asymmetric input
-    # quantisation over the row incl. the pack padding, zero point folded into the bias; ConvInt8TiledExecutor.cpp:1033, 1432, 2016-2050)
-    for (tokens, ic, oc, asym, hb, lo, hi) in [(8, 64, 48, False, True, -1, 1), (33, 256, 200, True, True, -1, 1),
-                                               (5, 96, 33, False, False, -1, 1), (64, 512, 128, True, False, -1, 1),
-                                               (1, 2048, 512, True, True, -1, 1), (1, 100, 64, False, False, 0.2, 1.0),
-                                               (1, 250, 33, True, False, -1, -0.1), (1, 320, 200, True, True, -3, 5),
-                                               (1, 64, 48, False, True, 0.25, 0.25)]:
-        x = rng.uniform(lo, hi, (tokens, ic)).astype(np.float32)
-        wq = rng.integers(-128, 128, (oc, ic)).astype(np.int8)
-        alpha = rng.uniform(0.001, 0.01, oc).astype(np.float32)
-        wmin = rng.uniform(-0.05, 0.05, oc).astype(np.float32) if asym else np.zeros(0, np.float32)
-        bias = rng.uniform(-1, 1, oc).astype(np.float32) if hb else np.zeros(0, np.float32)
+    """depthwise int8 conv + dynamic-quant linear outputs from the real reference (refdump conv mode 1 / linear); the inputs are
+    regenerated from their seed by tests/cases.dw_linear_inputs and not stored."""
+    g = dw_linear_inputs()
+    out = {"ndw": len(DW_CASES), "nlin": len(LINEAR_CASES)}
+    for i, (ch, k, n, ih, iw, st, pad, relu) in enumerate(DW_CASES):
+        s_in, z_in, s_out, z_out = g[f"d{i}_q"]
+        out[f"d{i}_y"] = O.ref_conv(1, g[f"d{i}_x"], g[f"d{i}_w"], g[f"d{i}_bias"], g[f"d{i}_ws"], stride=st, pad=pad, group=ch,
+                                    relu=relu, z_in=int(z_in), z_out=int(z_out), scale_in=s_in, scale_out=s_out)
+    for j, (tokens, ic, oc, asym, hb, lo, hi) in enumerate(LINEAR_CASES):
+        alpha, wmin, bias = g[f"l{j}_alpha"], g[f"l{j}_wmin"], g[f"l{j}_bias"]
         al = np.stack([wmin, alpha], 1).ravel() if asym else alpha
-        y = O.ref_linear(x, wq, al, asym=asym, bias=bias if hb else None)
-        out.update({f"l{j}_x": x, f"l{j}_wq": wq, f"l{j}_alpha": alpha, f"l{j}_wmin": wmin, f"l{j}_bias": bias, f"l{j}_y": y})
-        j += 1
-    out["nlin"] = j
+        out[f"l{j}_y"] = O.ref_linear(g[f"l{j}_x"], g[f"l{j}_wq"], al, asym=asym, bias=bias if hb else None)
     np.savez_compressed(os.path.join(HERE, "dw_linear_golden.npz"), **out)
-    print("dw_linear_golden.npz:", i, "depthwise,", j, "linear cases")
+    print("dw_linear_golden.npz:", len(DW_CASES), "depthwise,", len(LINEAR_CASES), "linear cases")
 
 
 def block_linear_golden():
@@ -147,7 +123,8 @@ def model_checkpoints():
     out = {}
     with tempfile.TemporaryDirectory() as d:
         recs = O.ref_run_model(model, 1, 7, d, 1)
-        out["input"] = np.fromfile(os.path.join(d, "input.f32"), np.float32).reshape(1, 3, 224, 224)
+        # the input is regenerated from the seed (tests/cases.refdump_input), not stored
+        assert np.array_equal(np.fromfile(os.path.join(d, "input.f32"), np.float32), refdump_input((1, 3, 224, 224), 7).ravel())
         names = []
         for r in recs:
             if r["name"] in keep and r["scale"] > 0:
@@ -188,20 +165,118 @@ def wino_golden():
 
 def matmul_golden():
     """float MatMul / BatchMatMul outputs of the real reference CPU backend (refdump matmul)."""
-    from tests.test_matmul import CASES, make
-    rng = np.random.default_rng(808)
+    from tests.test_matmul import CASES
+    g = matmul_inputs()        # regenerated from the seed, not stored
     out = {"ncase": len(CASES)}
-    for i, (bd, e, l, h, ta, tb) in enumerate(CASES):
-        a, b = make(rng, bd, e, l, h, ta, tb)
-        out.update({f"m{i}_a": a, f"m{i}_b": b, f"m{i}_ta": ta, f"m{i}_tb": tb, f"m{i}_y": O.ref_matmul(a, b, ta, tb)})
+    for i in range(len(CASES)):
+        out[f"m{i}_y"] = O.ref_matmul(g[f"m{i}_a"], g[f"m{i}_b"], bool(g[f"m{i}_ta"]), bool(g[f"m{i}_tb"]))
     np.savez_compressed(os.path.join(HERE, "matmul_golden.npz"), **out)
     print("matmul_golden.npz:", len(CASES), "cases")
 
 
+def reference_calls():
+    """The reference's answers to every request the oracle tests send it (conv, depthwise, linear, pool, matmul, Winograd):
+    tests/golden/reference_calls.npz, where oracle.py finds them by request when oracle/_ref is not built."""
+    from tests import test_matmul, test_oracle, test_winograd
+    O.recording = {}
+    for case in KAT_SWEEP[:5]:
+        test_oracle.test_oracle_bit_exact_vs_reference_legacy(case)
+    test_oracle.test_oracle_bit_exact_vs_reference_modern()
+    test_oracle.test_block_quant_linear_vs_live_reference()
+    test_oracle.test_single_token_linear_is_the_references_decode_arithmetic()
+    test_oracle.test_oracle_random_sweep_vs_live_reference()
+    test_oracle.test_int8_pool_oracle_vs_live_reference()
+    test_matmul.test_oracle_vs_live_reference()
+    test_winograd.test_oracle_bit_exact_vs_live_reference_avx2()
+    np.savez_compressed(O.RECORDED, **O.recording)
+    print("reference_calls.npz:", len(O.recording), "answers")
+    O.recording = None
+
+
+def scale_int8_golden():
+    """The first int8 Scale ops of ResNet-50 int8 (oracle/_ref/r50_int8.mnn, written by build()) as MNN_FORWARD_CPU runs them:
+    parameters, quant attrs and an 8x8 spatial crop of the int8 input and output (the op is per channel: a crop is a whole case)."""
+    import tempfile
+    from mnn_b200 import mnn_file
+    model = os.path.join(O.REF_DIR, "r50_int8.mnn")
+    net = mnn_file.load(model)
+    scales = [op for op in net.ops if op.type == "Scale"]
+    assert len(scales) == 17 and scales[0].attrs["scale"] is not None
+    out, k = {}, 0
+    with tempfile.TemporaryDirectory() as d:
+        by_name = {r["name"]: r for r in O.ref_run_model(model, 1, 3, d, 8)}
+        producers = {op.outputs[0]: op for op in net.ops if op.outputs}
+        for op in scales[:4]:
+            r_out, r_in = by_name.get(op.name), by_name.get(producers[op.inputs[0]].name)
+            if r_out is None or r_in is None or not r_out["apply_quant"] or not r_in["apply_quant"]:
+                continue
+            fi = np.fromfile(os.path.join(d, r_in["file"]), np.float32).reshape(r_in["dims"])
+            fo = np.fromfile(os.path.join(d, r_out["file"]), np.float32).reshape(r_out["dims"])
+            qi = np.rint(fi / np.float32(r_in["scale"]) + np.float32(r_in["zero"])).astype(np.int8)
+            qo = np.rint(fo / np.float32(r_out["scale"]) + np.float32(r_out["zero"])).astype(np.int8)
+            bias = op.attrs["bias"]
+            out.update({f"s{k}_name": op.name, f"s{k}_x": qi[:, :, :8, :8], f"s{k}_y": qo[:, :, :8, :8],
+                        f"s{k}_scale": np.asarray(op.attrs["scale"], np.float32),
+                        f"s{k}_bias": np.zeros(0, np.float32) if bias is None else np.asarray(bias, np.float32),
+                        f"s{k}_q": np.array([r_in["scale"], r_in["zero"], r_out["scale"], r_out["zero"], r_out["min"], r_out["max"]])})
+            k += 1
+    out["n"] = k
+    np.savez_compressed(os.path.join(HERE, "scale_int8_golden.npz"), **out)
+    print("scale_int8_golden.npz:", k, "ops")
+
+
+def fullsize_golden():
+    """What the reference computes at the bench configs' own sizes, as digests and samples (tests/test_gpu_wholenet.py,
+    tests/test_gpu_configs.py): every int8 tensor of MobileNet-v2 at batch 2 (sha256 of the codes) and at batch 32 (the harness's
+    position-weighted sums), the int8 Winograd F(6,3) outputs at batch 64 (sha256), the Qwen linear outputs at 4096 tokens
+    (max |y| and a fixed sample of positions)."""
+    import hashlib
+    import tempfile
+    from tests.cases import random_wino_case, refdump_input, wino_oracle
+    from tests.test_gpu_configs import MODEL, _refdump_run, c4_case, c4_sample_positions
+    from tests.test_gpu_wholenet import FP_INTERNAL
+    out = {}
+    with tempfile.TemporaryDirectory() as d:
+        recs = O.ref_run_model(MODEL, 2, 11, d, 8)
+        assert np.array_equal(np.fromfile(os.path.join(d, "input.f32"), np.float32), refdump_input((2, 3, 224, 224), 11).ravel())
+        names, digests = [], []
+        for r in recs:
+            if r["scale"] <= 0 or not r["apply_quant"]:
+                continue
+            f = np.fromfile(os.path.join(d, r["file"]), np.float32).reshape(r["dims"])
+            q = np.rint(f / np.float32(r["scale"]) + np.float32(r["zero"])).astype(np.int8)
+            names.append(r["name"])
+            digests.append(hashlib.sha256(q.tobytes()).hexdigest())
+            if r["name"] in FP_INTERNAL:
+                out[f"every_op_{r['name']}"] = q
+        out["every_op_names"], out["every_op_sha256"] = np.array(names), np.array(digests)
+    with tempfile.TemporaryDirectory() as d:
+        cpu, _ = _refdump_run(O.REFDUMP, O.REF_DIR, MODEL, 32, 5, d, min(os.cpu_count() or 1, 32), False)
+        assert np.array_equal(np.fromfile(os.path.join(d, "input.f32"), np.float32), refdump_input((32, 3, 224, 224), 5).ravel())
+        for key, field in (("names", "name"), ("types", "type"), ("hashes", "file"), ("scales", "scale"), ("zeros", "zero"),
+                           ("apply_quant", "apply_quant")):
+            out["c2_" + key] = np.array([r[field] for r in cpu])
+        out["c2_dims"] = np.array([",".join(str(v) for v in r["dims"]) for r in cpu])
+    for C_, HW in ((64, 56), (512, 7)):
+        c = random_wino_case(np.random.default_rng(C_ + HW), 6, 64, C_, C_, HW, HW, 1, True)
+        ref = np.ascontiguousarray(wino_oracle(O, c, 6, O.ref_wino), np.int8)
+        out[f"c3_{C_}_{HW}_sha256"] = np.array(hashlib.sha256(ref.tobytes()).hexdigest())
+    for ic, oc, asym, has_bias in ((2048, 6144, True, True), (5504, 2048, True, False)):
+        x, wq, alpha, wmin, bias = c4_case(4096, ic, oc, asym, has_bias)
+        al = np.stack([wmin, alpha], 1).astype(np.float32).ravel() if asym else alpha
+        ref = O.ref_linear(x, wq, al, asym=asym, bias=bias, threads=min(os.cpu_count() or 1, 32))
+        out[f"c4_{ic}_{oc}_sample"] = ref.ravel()[c4_sample_positions(4096, oc)]
+        out[f"c4_{ic}_{oc}_absmax"] = np.abs(ref).max()
+    np.savez_compressed(os.path.join(HERE, "reference_fullsize.npz"), **out)
+    print("reference_fullsize.npz:", len(out), "entries")
+
+
 if __name__ == "__main__":
-    # python tests/golden/make_golden.py [conv] [dw_linear] [block_linear] [hashes] [checkpoints] [wino] [matmul]   (default: all)
+    # python tests/golden/make_golden.py [conv] [dw_linear] [block_linear] [hashes] [checkpoints] [wino] [matmul] [calls] [scale]
+    #                                    [fullsize]   (default: all)
     assert O.have_reference(), "build oracle/_ref first: python oracle/build_ref.py"
-    which = set(sys.argv[1:]) or {"conv", "dw_linear", "block_linear", "hashes", "checkpoints", "wino", "matmul"}
+    which = set(sys.argv[1:]) or {"conv", "dw_linear", "block_linear", "hashes", "checkpoints", "wino", "matmul", "calls", "scale",
+                                  "fullsize"}
     if "conv" in which:
         conv_golden()
     if "dw_linear" in which:
@@ -216,3 +291,9 @@ if __name__ == "__main__":
         wino_golden()
     if "matmul" in which:
         matmul_golden()
+    if "calls" in which:
+        reference_calls()
+    if "scale" in which:
+        scale_int8_golden()
+    if "fullsize" in which:
+        fullsize_golden()

@@ -6,7 +6,7 @@ import numpy as np
 import pytest
 
 from oracle import oracle as O
-from tests.cases import KAT_SWEEP, kat_conv, random_modern_case
+from tests.cases import KAT_SWEEP, kat_conv, load_golden, random_modern_case
 
 pytestmark = pytest.mark.gpu
 GOLD = os.path.join(os.path.dirname(__file__), "golden")
@@ -198,7 +198,7 @@ def test_depthwise_and_linear_golden_fixtures(backend):
     import torch
     from mnn_b200.backend import Op, QuantAttr, Tensor
     from tests.test_oracle import wire_wzero
-    g = np.load(os.path.join(GOLD, "dw_linear_golden.npz"))
+    g = load_golden("dw_linear_golden")
     for i in range(int(g["ndw"])):
         s_in, z_in, s_out, z_out = g[f"d{i}_q"]
         x, w = g[f"d{i}_x"], g[f"d{i}_w"]

@@ -1,12 +1,13 @@
 """GPU: the whole MobileNet-v2 int8 .mnn on the CUDA path (no CPU fallback) against the REAL reference CPU backend:
-committed checkpoints always, every op live when oracle/_ref is present on the box."""
+committed checkpoints at batch 1, and every op at batch 2 against the digests of the reference's own dump
+(tests/golden/reference_fullsize.npz, recorded by tests/golden/make_golden.py)."""
+import hashlib
 import os
-import tempfile
 
 import numpy as np
 import pytest
 
-from oracle import oracle as O
+from tests.cases import load_golden, refdump_input
 
 pytestmark = pytest.mark.gpu
 GOLD = os.path.join(os.path.dirname(__file__), "golden")
@@ -17,7 +18,7 @@ FP_INTERNAL = ("MobilenetV2/Predictions/Softmax",)
 
 def test_wholenet_checkpoints_vs_reference_golden():
     from mnn_b200.session import WholeNetSession
-    g = np.load(os.path.join(GOLD, "mbv2_int8_checkpoints.npz"))
+    g = load_golden("mbv2_int8_checkpoints")
     sess = WholeNetSession(MODEL, 1)
     sess.set_input(g["input"])
     sess.run()
@@ -33,53 +34,49 @@ def test_wholenet_checkpoints_vs_reference_golden():
     assert np.abs(out - ref).max() <= 1e-3 * max(np.abs(ref).max(), 1e-6) + 0.05   # one softmax LSB = scale ~0.03
 
 
-@pytest.mark.skipif(not O.have_reference(), reason="oracle/_ref not on this box")
+def _check_every_op(sess, g, what=""):
+    """every int8 tensor of the reference's per-command dump (batch 2, input seed 11, quantised with the tensor's own attrs)
+    against the session's checkpoint of the same name: bit-exact (sha256 of the int8 codes), softmax within 1 LSB"""
+    checked = 0
+    for name, digest in zip(g["every_op_names"], g["every_op_sha256"]):
+        name = str(name)
+        if name not in sess.checkpoints:
+            continue
+        got = np.ascontiguousarray(sess.read_int8(name), np.int8)
+        if name in FP_INTERNAL:
+            ref = g[f"every_op_{name}"].reshape(got.shape)
+            dmax = np.abs(got.astype(int) - ref.astype(int)).max()
+            assert dmax <= 1, f"{what}{name}: max |diff| = {dmax}"
+        else:
+            assert hashlib.sha256(got.tobytes()).hexdigest() == str(digest), f"{what}{name}: differs from the reference"
+        checked += 1
+    assert checked >= 60, checked       # 36 conv + 17 depthwise + 10 add + pool + softmax
+
+
 @pytest.mark.parametrize("batch", [2])
 def test_wholenet_every_op_vs_live_reference(batch):
+    """every int8 tensor against the reference CPU backend's own per-command dump of the same input (recorded digests)"""
     from mnn_b200.session import WholeNetSession
-    with tempfile.TemporaryDirectory() as d:
-        recs = O.ref_run_model(MODEL, batch, 11, d, 8)
-        x = np.fromfile(os.path.join(d, "input.f32"), np.float32).reshape(batch, 3, 224, 224)
-        sess = WholeNetSession(MODEL, batch)
-        sess.capture()                      # CUDA-graph replay is the product path
-        sess.set_input(x)
-        sess.run()
-        checked = 0
-        for r in recs:
-            if r["name"] not in sess.checkpoints or r["scale"] <= 0 or not r["apply_quant"]:
-                continue
-            f = np.fromfile(os.path.join(d, r["file"]), np.float32).reshape(r["dims"])
-            q = np.rint(f / np.float32(r["scale"]) + np.float32(r["zero"])).astype(np.int8)
-            got = sess.read_int8(r["name"])
-            dmax = np.abs(got.astype(int) - q.reshape(got.shape).astype(int)).max()
-            assert dmax <= (1 if r["name"] in FP_INTERNAL else 0), f"{r['name']}: max |diff| = {dmax}"
-            checked += 1
-        assert checked >= 60, checked       # 36 conv + 17 depthwise + 10 add + pool + softmax
+    g = np.load(os.path.join(GOLD, "reference_fullsize.npz"))
+    x = refdump_input((batch, 3, 224, 224), 11)
+    sess = WholeNetSession(MODEL, batch)
+    sess.capture()                      # CUDA-graph replay is the product path
+    sess.set_input(x)
+    sess.run()
+    _check_every_op(sess, g)
 
 
-@pytest.mark.skipif(not O.have_reference(), reason="oracle/_ref not on this box")
 def test_wholenet_program_mode_every_op_vs_live_reference():
     """The same .mnn with its conv / depthwise / add chain fused into ONE cooperative launch (net program: dependency flags between
-    tiles of consecutive layers): every checkpoint still equals the live reference, twice in a row (flags are re-armed per launch)."""
+    tiles of consecutive layers): every checkpoint still equals the reference, twice in a row (flags are re-armed per launch)."""
     from mnn_b200.session import WholeNetSession
     batch = 2
-    with tempfile.TemporaryDirectory() as d:
-        recs = O.ref_run_model(MODEL, batch, 11, d, 8)
-        x = np.fromfile(os.path.join(d, "input.f32"), np.float32).reshape(batch, 3, 224, 224)
-        sess = WholeNetSession(MODEL, batch, program=True)
-        assert sess.programs and sess.launches_per_step <= 12, [s[0] for s in sess.steps]
-        sess.capture()
-        for rep in range(2):
-            sess.set_input(x)
-            sess.run()
-            checked = 0
-            for r in recs:
-                if r["name"] not in sess.checkpoints or r["scale"] <= 0 or not r["apply_quant"]:
-                    continue
-                f = np.fromfile(os.path.join(d, r["file"]), np.float32).reshape(r["dims"])
-                q = np.rint(f / np.float32(r["scale"]) + np.float32(r["zero"])).astype(np.int8)
-                got = sess.read_int8(r["name"])
-                dmax = np.abs(got.astype(int) - q.reshape(got.shape).astype(int)).max()
-                assert dmax <= (1 if r["name"] in FP_INTERNAL else 0), f"rep {rep} {r['name']}: max |diff| = {dmax}"
-                checked += 1
-            assert checked >= 60, checked
+    g = np.load(os.path.join(GOLD, "reference_fullsize.npz"))
+    x = refdump_input((batch, 3, 224, 224), 11)
+    sess = WholeNetSession(MODEL, batch, program=True)
+    assert sess.programs and sess.launches_per_step <= 12, [s[0] for s in sess.steps]
+    sess.capture()
+    for rep in range(2):
+        sess.set_input(x)
+        sess.run()
+        _check_every_op(sess, g, f"rep {rep} ")

@@ -6,9 +6,8 @@ import numpy as np
 import pytest
 
 from oracle import oracle as O
+from tests.cases import load_golden
 
-GOLD = os.path.join(os.path.dirname(__file__), "golden", "matmul_golden.npz")
-needs_ref = pytest.mark.skipif(not O.have_reference(), reason="oracle/_ref not built")
 # (batch dims, e, l, h, transpose_a, transpose_b): attention QK^T / PV of Qwen-1.8B (16 heads x 128), plus ragged shapes
 CASES = [((2, 4), 64, 128, 64, False, True), ((3,), 64, 64, 128, False, False), ((), 37, 53, 29, False, False),
          ((), 40, 24, 56, True, False), ((2,), 33, 72, 17, True, True), ((), 1, 200, 300, False, True)]
@@ -23,15 +22,13 @@ def make(rng, bd, e, l, h, ta, tb, positive=False):
 
 
 def test_oracle_vs_golden_fixture():
-    g = np.load(GOLD)
+    g = load_golden("matmul_golden")
     for i in range(int(g["ncase"])):
         y = O.matmul_f32(g[f"m{i}_a"], g[f"m{i}_b"], bool(g[f"m{i}_ta"]), bool(g[f"m{i}_tb"]))
         ref = g[f"m{i}_y"]
         assert y.shape == ref.shape and np.abs(y - ref).max() <= 1e-5 * np.abs(ref).max()
 
 
-@needs_ref
-@pytest.mark.reference
 def test_oracle_vs_live_reference():
     rng = np.random.default_rng(3)
     for bd, e, l, h, ta, tb in CASES[:4]:
@@ -59,7 +56,7 @@ def run_matmul(backend, a, b, ta, tb, bias=None):
 
 @pytest.mark.gpu
 def test_gpu_vs_golden_and_oracle(backend):
-    g = np.load(GOLD)
+    g = load_golden("matmul_golden")
     for i in range(int(g["ncase"])):
         y = run_matmul(backend, g[f"m{i}_a"], g[f"m{i}_b"], bool(g[f"m{i}_ta"]), bool(g[f"m{i}_tb"]))
         ref = g[f"m{i}_y"]

@@ -1,16 +1,15 @@
 """CPU tests (-m "not gpu"): the oracle against the reference's known-answer generators, the committed golden
-fixtures and -- when oracle/_ref exists (this container; the GPU box gets the prebuilt files) -- against the
-UNMODIFIED reference CPU backend itself, bit for bit."""
+fixtures and the UNMODIFIED reference CPU backend itself, bit for bit: live where oracle/_ref is built, elsewhere its answers to the same
+requests as recorded in tests/golden/reference_calls.npz (the *_live_reference tests)."""
 import os
 
 import numpy as np
 import pytest
 
 from oracle import oracle as O
-from tests.cases import KAT_SWEEP, kat_conv, random_modern_case
+from tests.cases import KAT_SWEEP, kat_conv, load_golden, random_modern_case
 
 GOLD = os.path.join(os.path.dirname(__file__), "golden")
-needs_ref = pytest.mark.skipif(not O.have_reference(), reason="oracle/_ref not built")
 
 
 def naive_conv_int8(x, w, bias, scale, stride, pad, dilate):
@@ -64,7 +63,6 @@ def test_oracle_vs_golden_fixtures():
         assert np.array_equal(y, p["y"]), f"golden case {i} differs"
 
 
-@needs_ref
 @pytest.mark.parametrize("case", KAT_SWEEP[:5])
 def test_oracle_bit_exact_vs_reference_legacy(case):
     (ic, oc), (kh, kw), n, pad, stride, dilate, (ih, iw) = case
@@ -75,7 +73,6 @@ def test_oracle_bit_exact_vs_reference_legacy(case):
     assert np.array_equal(yr, yo)
 
 
-@needs_ref
 def test_oracle_bit_exact_vs_reference_modern():
     rng = np.random.default_rng(11)
     for (ic, oc, kh, kw, n, st, pad, relu) in [(3, 32, 3, 3, 2, (2, 2), (1, 1), 1), (16, 24, 1, 1, 3, (1, 1), (0, 0), 0),
@@ -106,7 +103,7 @@ def wire_wzero(wmin, alpha):
 
 
 def test_depthwise_and_linear_vs_golden_fixtures():
-    g = np.load(os.path.join(GOLD, "dw_linear_golden.npz"))
+    g = load_golden("dw_linear_golden")
     for i in range(int(g["ndw"])):
         s_in, z_in, s_out, z_out = g[f"d{i}_q"]
         relu = int(g[f"d{i}_relu"])
@@ -143,8 +140,6 @@ def test_block_quant_linear_vs_golden_fixtures():
     assert np.array_equal(O.linear_w8_dynamic(x[:1], wq, alpha), O.linear_w8_dynamic_blocks(x[:1], wq, alpha, None, None, 1))
 
 
-@needs_ref
-@pytest.mark.reference
 def test_block_quant_linear_vs_live_reference():
     rng = np.random.default_rng(12)
     for (tokens, ic, oc, blocks, asym, hb) in [(2, 128, 48, 2, True, True), (17, 640, 64, 5, False, False), (1, 320, 72, 5, True, True)]:
@@ -160,8 +155,6 @@ def test_block_quant_linear_vs_live_reference():
         assert np.abs(y - ref).max() / np.abs(ref).max() < 4e-6
 
 
-@needs_ref
-@pytest.mark.reference
 def test_single_token_linear_is_the_references_decode_arithmetic():
     """ONE token takes a different path in the reference (asymmetric single-quant with the input zero folded into the bias) than
     two or more (symmetric per-token quant): the restatement follows both, and the two differ by far more than the tolerance."""
@@ -182,8 +175,6 @@ def test_single_token_linear_is_the_references_decode_arithmetic():
         assert np.abs(two - ref).max() / np.abs(ref).max() > 1e-4
 
 
-@needs_ref
-@pytest.mark.reference
 def test_oracle_random_sweep_vs_live_reference():
     """A seeded random sweep of the restatement against the UNMODIFIED reference CPU backend (conv modern form through a
     real 2-op .mnn, conv legacy form, depthwise): kernel sizes, strides, pads, dilations, ragged channels, zero points."""
@@ -230,8 +221,6 @@ POOL_CASES = [(1, 16, 8, 8, (3, 3), (2, 2), (1, 1), 1), (2, 20, 9, 7, (2, 2), (2
               (1, 8, 10, 10, (3, 3), (1, 1), (1, 1), 0), (1, 5, 6, 9, (3, 2), (1, 2), (1, 0), 1), (3, 64, 12, 12, (3, 3), (2, 2), (1, 1), 0)]
 
 
-@needs_ref
-@pytest.mark.reference
 def test_int8_pool_oracle_vs_live_reference():
     """int8 pooling with equal in/out quant attrs (kept in int8 by the CPU's onSetQuantInfo): the restatement of the x86
     kernels -- average on the uint8 storage with a 2^24 fixed-point reciprocal, MAX comparing the stored bytes as signed --
@@ -252,35 +241,16 @@ def test_int8_pool_oracle_vs_live_reference():
     assert differs_from_true_max
 
 
-@pytest.mark.skipif(not (O.have_reference() and os.path.exists(os.path.join(O.REF_DIR, "r50_int8.mnn"))),
-                    reason="oracle/_ref (reference build + ResNet-50 fixture) not present")
 def test_scale_int8_oracle_pinned_on_live_reference():
     """The numpy restatement of CPUScaleInt8 + MNNScaleAndAddBiasInt8 against the REAL reference: the first int8 Scale ops of
-    ResNet-50 int8 (oracle/_ref/r50_int8.mnn) as executed by MNN_FORWARD_CPU, input and output tensors taken from the
-    per-command dump of `refdump run`."""
-    import tempfile
-    from mnn_b200 import mnn_file
-    model = os.path.join(O.REF_DIR, "r50_int8.mnn")
-    net = mnn_file.load(model)
-    scales = [op for op in net.ops if op.type == "Scale"]
-    assert len(scales) == 17 and scales[0].attrs["scale"] is not None
-    with tempfile.TemporaryDirectory() as d:
-        recs = O.ref_run_model(model, 1, 3, d, 8)
-        by_name = {r["name"]: r for r in recs}
-        producers = {op.outputs[0]: op for op in net.ops if op.outputs}
-        checked = 0
-        for op in scales[:4]:
-            r_out = by_name.get(op.name)
-            src = producers[op.inputs[0]]
-            r_in = by_name.get(src.name)
-            if r_out is None or r_in is None or not r_out["apply_quant"] or not r_in["apply_quant"]:
-                continue
-            fi = np.fromfile(os.path.join(d, r_in["file"]), np.float32).reshape(r_in["dims"])
-            fo = np.fromfile(os.path.join(d, r_out["file"]), np.float32).reshape(r_out["dims"])
-            qi = np.rint(fi / np.float32(r_in["scale"]) + np.float32(r_in["zero"])).astype(np.int8)
-            qo = np.rint(fo / np.float32(r_out["scale"]) + np.float32(r_out["zero"])).astype(np.int8)
-            y = O.scale_int8(qi, op.attrs["scale"], op.attrs["bias"], r_in["scale"], int(r_in["zero"]), r_out["scale"], int(r_out["zero"]),
-                             int(r_out["min"]), int(r_out["max"]))
-            assert np.array_equal(y, qo), (op.name, np.abs(y.astype(int) - qo.astype(int)).max())
-            checked += 1
-        assert checked >= 3
+    ResNet-50 int8 (oracle/_ref/r50_int8.mnn) as executed by MNN_FORWARD_CPU, recorded from the per-command dump of `refdump run`
+    (tests/golden/scale_int8_golden.npz: each op's parameters and quant attrs, an 8x8 spatial crop of its int8 input and output)."""
+    g = np.load(os.path.join(GOLD, "scale_int8_golden.npz"))
+    assert int(g["n"]) >= 3
+    for k in range(int(g["n"])):
+        s_in, z_in, s_out, z_out, min_v, max_v = g[f"s{k}_q"]
+        bias = g[f"s{k}_bias"]
+        y = O.scale_int8(g[f"s{k}_x"], g[f"s{k}_scale"], bias if bias.size else None, s_in, int(z_in), s_out, int(z_out),
+                         int(min_v), int(max_v))
+        qo = g[f"s{k}_y"]
+        assert np.array_equal(y, qo), (str(g[f"s{k}_name"]), np.abs(y.astype(int) - qo.astype(int)).max())

@@ -1,6 +1,6 @@
 """The drop-in boundary, end to end (-m gpu): the UNMODIFIED reference core (oracle/_ref/libMNN.so: Interpreter, Session,
 Pipeline, geometry, quant-cast insertion) schedules tests/golden/mbv2_int8.mnn on MNN_FORWARD_CUDA, where the only registered
-RuntimeCreator is mnn_b200/libmnn_b200_plugin.so (mnn_b200/csrc/plugin/b200_plugin.cpp -> C ABI -> sm_100a kernels).  Every
+RuntimeCreator is oracle/_ref/libmnn_b200_plugin.so (mnn_b200/csrc/plugin/b200_plugin.cpp -> C ABI -> sm_100a kernels).  Every
 command's output tensor, read back through the plugin's onCopyBuffer, must equal what the same process produces on
 MNN_FORWARD_CPU -- bit for bit for int8 tensors (compared at the dequantised boundary, SURVEY F6), and the plugin must have
 created EVERY command (nothing handed back to the CPU backup backend)."""
@@ -13,16 +13,18 @@ import numpy as np
 import pytest
 
 from oracle import oracle as O
+from tests.cases import load_golden
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-PLUGIN = os.path.join(ROOT, "mnn_b200", "libmnn_b200_plugin.so")
+PLUGIN = O.PLUGIN
 MODEL = os.path.join(ROOT, "tests", "golden", "mbv2_int8.mnn")
 
 
 def test_plugin_library_is_built_and_exports_registration_hook():
     """CPU-side check: the plugin .so exists in-tree and exports its stats hook; it links the C ABI library."""
-    if not os.path.exists(PLUGIN):
-        pytest.skip("plugin not built (needs the reference headers: python mnn_b200/csrc/plugin/build_plugin.py)")
+    if not O.have_reference():
+        pytest.skip("the plugin is built with the reference core (oracle/_ref), which is not built here")
+    assert os.path.exists(PLUGIN), "the plugin is missing although the reference core is built (mnn_b200/csrc/plugin/build_plugin.py)"
     out = subprocess.run(["nm", "-D", "--defined-only", PLUGIN], capture_output=True, text=True, check=True).stdout
     assert "mnnb200_plugin_stats" in out
     need = subprocess.run(["objdump", "-p", PLUGIN], capture_output=True, text=True, check=True).stdout
@@ -53,10 +55,7 @@ def _run(outdir, batch, plugin, model=None):
 @pytest.mark.gpu
 @pytest.mark.parametrize("batch", [1, 4])
 def test_reference_pipeline_on_plugin_matches_cpu_backend(batch):
-    if not O.have_reference():
-        pytest.skip("the reference core (oracle/_ref, built from /root/reference by oracle/build_ref.py) is not in this snapshot")
-    if not os.path.exists(PLUGIN):
-        pytest.fail("mnn_b200/libmnn_b200_plugin.so is missing although the reference core is present")
+    _need_ref_and_plugin()
     with tempfile.TemporaryDirectory() as d:
         cpu, _, _ = _run(os.path.join(d, "cpu"), batch, False)
         gpu, stats, r = _run(os.path.join(d, "gpu"), batch, True)
@@ -81,9 +80,9 @@ def test_reference_pipeline_on_plugin_matches_cpu_backend(batch):
 
 def _need_ref_and_plugin():
     if not O.have_reference():
-        pytest.skip("the reference core (oracle/_ref) is not in this snapshot")
+        pytest.skip("the reference core (oracle/_ref, built by oracle/build_ref.py) is not built here")
     if not os.path.exists(PLUGIN):
-        pytest.fail("mnn_b200/libmnn_b200_plugin.so is missing although the reference core is present")
+        pytest.fail("oracle/_ref/libmnn_b200_plugin.so is missing although the reference core is present")
 
 
 def _plugin_env():
@@ -99,7 +98,7 @@ def test_llm_linear_through_reference_executor_on_plugin():
     outputs the reference CPU backend recorded in tests/golden/dw_linear_golden.npz."""
     import struct
     _need_ref_and_plugin()
-    g = np.load(os.path.join(ROOT, "tests", "golden", "dw_linear_golden.npz"))
+    g = load_golden("dw_linear_golden")
     for j in range(int(g["nlin"])):
         x, wq, alpha, wmin, bias, ref = (g[f"l{j}_{k}"] for k in ("x", "wq", "alpha", "wmin", "bias", "y"))
         tokens, ic = x.shape
@@ -124,7 +123,7 @@ def test_llm_linear_through_reference_executor_on_plugin():
 def test_matmul_through_reference_executor_on_plugin():
     import struct
     _need_ref_and_plugin()
-    g = np.load(os.path.join(ROOT, "tests", "golden", "matmul_golden.npz"))
+    g = load_golden("matmul_golden")
     done = 0
     for i in range(int(g["ncase"])):
         a, b, ta, tb, ref = g[f"m{i}_a"], g[f"m{i}_b"], bool(g[f"m{i}_ta"]), bool(g[f"m{i}_tb"]), g[f"m{i}_y"]
@@ -187,7 +186,7 @@ def test_resnet50_int8_on_plugin_matches_cpu_backend(model_name):
     _need_ref_and_plugin()
     model = os.path.join(O.REF_DIR, model_name)
     if not os.path.exists(model):
-        pytest.skip(f"{model_name} not generated (python -c 'import __graft_entry__ as g; g.build()' where /root/reference exists)")
+        pytest.skip(f"{model_name} not generated (build() writes it where the reference sources are present)")
     batch = 2
     with tempfile.TemporaryDirectory() as d:
         cpu, _, _ = _run(os.path.join(d, "cpu"), batch, False, model)

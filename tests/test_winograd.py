@@ -9,7 +9,6 @@ from oracle import oracle as O
 from tests.cases import kat_wino, random_wino_case, wino_oracle
 
 GOLD = os.path.join(os.path.dirname(__file__), "golden", "wino_int8_golden.npz")
-needs_ref2 = pytest.mark.skipif(not O.have_reference_avx2(), reason="oracle/_ref/refdump_avx2 not built")
 
 
 def golden_cases():
@@ -52,8 +51,6 @@ def test_oracle_close_to_direct_float_conv():
         assert np.abs(y - refc).mean() < 8.0 and np.corrcoef(y.ravel(), refc.ravel())[0, 1] > 0.9
 
 
-@needs_ref2
-@pytest.mark.reference
 def test_oracle_bit_exact_vs_live_reference_avx2():
     rng = np.random.default_rng(99)
     c = kat_wino(3, 32, 32, 39, 47)       # the reference unit test's exact configuration, batch 3

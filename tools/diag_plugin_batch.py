@@ -4,7 +4,7 @@ import numpy as np
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
 from oracle import oracle as O
-PLUGIN = os.path.join(ROOT, "mnn_b200", "libmnn_b200_plugin.so")
+PLUGIN = os.path.join(ROOT, "oracle", "_ref", "libmnn_b200_plugin.so")
 MODEL = os.path.join(ROOT, "tests", "golden", "mbv2_int8.mnn")
 
 def run(outdir, batch, plugin, extra=None, ncmd=3):
